@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the SkellySim hydrodynamic hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2|c4] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -29,6 +29,8 @@ matvecs (a slice of one GMRES solve), so that the driver's 20 steps time ~2 s of
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU port of the reference's OpenMP direct path for the
 same matvec (oracle/, all host threads; PVFMM/STKFMM/Eigen are not installable here); ranks > 0 exit at once.
+`--dump-outputs DIR` writes the result of the last timed matvec (res_fibers, res_shell, v_bodies; float64 .npy) so that
+two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -619,6 +621,31 @@ def accuracy_gate(rs: RankSystem, n_fibers_checked=48, n_shell_checked=1536, n_b
             "targets_checked": int(rows.shape[0]), "fibers_checked": int(len(fib_sel)), "gate": 1e-12}
 
 
+def dump_outputs(rs: RankSystem, out_dir: str):
+    """--dump-outputs: the result of the last matvec of the timed device path, i.e. what skb_flow_apply_matvec_device
+    hands its caller (res_fibers (4 N_f,), res_shell (N_s, 3) -- v_shell without the dense operator -- and v_bodies
+    (N_b, 3)), assembled over the ranks, written by rank 0 as out_dir/<name>.npy in float64.  Geometry, operators and
+    inputs are seeded, so two builds can be compared file by file.  Whole arrays: the largest workload (c4) writes 32 MB.
+    Rows no rank owns would stay NaN."""
+    rs.torch.cuda.synchronize()
+    parts = [(rs.ranges, rs.d_res.cpu().numpy()[:4 * rs.n_fw], rs.d_outs.cpu().numpy()[:rs.n_sw],
+              rs.d_vb.cpu().numpy()[:rs.n_bw])]
+    if rs.world > 1:
+        import torch.distributed as dist
+        mine, parts = parts[0], [None] * rs.world
+        dist.all_gather_object(parts, mine)
+    if rs.rank != 0:
+        return
+    n = rs.g["n"]
+    res, shell, body = np.full(4 * rs.nf, np.nan), np.full((rs.ns, 3), np.nan), np.full((rs.nb, 3), np.nan)
+    for (f0, f1, s0, s1, b0, b1), r, s, b in parts:
+        res[4 * n * f0:4 * n * f1], shell[s0:s1], body[b0:b1] = r, s, b
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "res_fibers.npy"), res)
+    np.save(os.path.join(out_dir, "res_shell.npy" if rs.dn is not None else "v_shell.npy"), shell)
+    np.save(os.path.join(out_dir, "v_bodies.npy"), body)
+
+
 # ------------------------------------------------------------------------------------------------
 # extra legs (N = 1)
 # ------------------------------------------------------------------------------------------------
@@ -873,7 +900,13 @@ def main():
     ap.add_argument("--no-dense-leg", action="store_true")
     ap.add_argument("--no-inprocess", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's matvec result as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.exchange == "nccl":
+        ap.error("--dump-outputs: the --exchange nccl A/B path keeps no result buffers")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -963,6 +996,8 @@ def main():
         n0 = capi.launch_count()
         tot_ms, wall = timed(step_device, args.steps, sample_sym=True)
         launches = capi.launch_count() - n0
+    if args.dump_outputs:  # before the e2e pass, which reuses the device buffers
+        dump_outputs(rs, args.dump_outputs)
     e2e_ms, _ = timed(step_e2e, args.steps)
     missing = rs.fl.group_error() if world > 1 and args.exchange == "peer" else -1
 

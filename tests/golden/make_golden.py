@@ -10,11 +10,14 @@ Imports the reference's own Green's-function kernels, `src/skelly_sim/kernels.py
 `rotlet_kernel_source_target_numba` :335-384), evaluates them on seeded inputs and stores
 inputs + outputs as small .npz fixtures next to this script.  The numba kernels regularise
 r < 1e-5 instead of skipping r == 0, so every case keeps sources and targets non-coincident
-(min separation asserted below); coincident-point semantics are pinned on the GPU box against
-the reference's CUDA kernels (oracle/_ref/libskelly_ref_kernels_cu.so).
+(min separation asserted below); coincident-point semantics are pinned by a fourth fixture,
+the outputs of the reference's CUDA kernels (oracle/_ref/libskelly_ref_kernels_cu.so, built by
+`make -C oracle` from the reference tree), generated on a GPU with
+
+    python tests/golden/make_golden.py --cuda
 
 The fixtures are the reference's outputs: tests compare the oracle (and through it the CUDA path)
-against them; nothing at test time reads /root/reference.
+against them; nothing at test time reads the reference tree or its build.
 """
 import importlib.util
 import os
@@ -166,7 +169,31 @@ def shell_double_layer():
     print(f"shell_double_layer: {n} nodes -> {os.path.basename(out)} ({os.path.getsize(out)} B)")
 
 
+def reference_cuda():
+    """Fourth fixture: kernels::stokeslet_direct_gpu_impl / stresslet_direct_gpu_impl of the reference's kernels.cu,
+    compiled unmodified, on the kernel_test.cpp shape (1229 sources, 743 targets) with 17 targets ON sources: the
+    r == 0 pairs the numba kernels cannot pin (they regularise) contribute exactly 0 here."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    import oracle as orc
+    if not orc.refgpu_available():
+        sys.exit("oracle/_ref/libskelly_ref_kernels_cu.so not built: run `make -C oracle` with the reference tree")
+    rng = np.random.default_rng(21)
+    r_src = rng.uniform(-1, 1, (1229, 3))
+    r_trg = rng.uniform(-1, 1, (743, 3))
+    r_trg[:17] = r_src[:17]
+    f_sl, f_dl = rng.uniform(-1, 1, (1229, 3)), rng.uniform(-1, 1, (1229, 9))
+    u_sl = orc.ref_stokeslet_direct_gpu_impl(r_src, f_sl, r_trg)
+    u_dl = orc.ref_stresslet_direct_gpu_impl(r_src, f_dl, r_trg)
+    out = os.path.join(HERE, "ref_cuda_kernels.npz")
+    np.savez_compressed(out, r_src=r_src, r_trg=r_trg, f_sl=f_sl, f_dl=f_dl, u_stokeslet=u_sl, u_stresslet=u_dl)
+    print(f"reference_cuda: n_src={r_src.shape[0]} n_trg={r_trg.shape[0]} -> {os.path.basename(out)} "
+          f"({os.path.getsize(out)} B)")
+
+
 if __name__ == "__main__":
+    if sys.argv[1:] == ["--cuda"]:
+        reference_cuda()
+        sys.exit(0)
     if not os.path.exists(REF):
         sys.exit("reference tree not present: golden vectors can only be regenerated in the build container")
     main()

@@ -44,6 +44,28 @@ def test_reference_kernel_only_figure_is_read_from_the_committed_launch_list(tmp
     assert bench.ref_kernel_only_ms(str(p)) is None
 
 
+def test_dump_outputs_writes_the_result_buffers_as_float64_npy(tmp_path):
+    """--dump-outputs on one rank: each result buffer trimmed to the rows the rank owns, one .npy per array."""
+    import types
+
+    import torch
+    g = bench.make_system("c3", 1, sizes=(3, 20, 5, 1, "weak"))
+    nf, ns, nb = g["fib"].shape[0], g["shell"].shape[0], g["body"].shape[0]
+    rng = np.random.default_rng(0)
+    res, outs, vb = rng.normal(size=4 * nf + 1), rng.normal(size=(ns + 1, 3)), rng.normal(size=(nb + 1, 3))
+    rs = types.SimpleNamespace(torch=types.SimpleNamespace(cuda=types.SimpleNamespace(synchronize=lambda: None)),
+                               g=g, world=1, rank=0, ranges=(0, 3, 0, ns, 0, nb), nf=nf, ns=ns, nb=nb, n_fw=nf, n_sw=ns,
+                               n_bw=nb, dn=object(), d_res=torch.from_numpy(res), d_outs=torch.from_numpy(outs),
+                               d_vb=torch.from_numpy(vb))
+    bench.dump_outputs(rs, str(tmp_path / "out"))
+    got = {p.name: np.load(p) for p in (tmp_path / "out").iterdir()}
+    assert sorted(got) == ["res_fibers.npy", "res_shell.npy", "v_bodies.npy"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["res_fibers.npy"], res[:4 * nf])
+    assert np.array_equal(got["res_shell.npy"], outs[:ns])
+    assert np.array_equal(got["v_bodies.npy"], vb[:nb])
+
+
 def test_cpu_arm_matches_the_plain_oracle_on_a_small_system():
     """CpuMatvec (what `--impl reference`, `cpu_baseline` and the in-run accuracy gate use: threaded C kernels + batched
     numpy) == the loop-form oracle composition of System::apply_matvec (oracle.apply_matvec_fibers, system.cpp:298-319),

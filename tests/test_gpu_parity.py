@@ -1,14 +1,16 @@
 """GPU parity tests (run with -m gpu on a B200): the CUDA path, called through the C ABI, against the CPU
-oracle, the committed golden fixtures (reference numba outputs) and the reference's own CUDA kernels
-(oracle/_ref/libskelly_ref_kernels_cu.so, compiled unmodified from src/core/kernels.cu).
+oracle, the committed golden fixtures (reference numba outputs) and the stored outputs of the reference's own CUDA
+kernels (src/core/kernels.cu compiled unmodified, tests/golden/ref_cuda_kernels.npz).
 
 Tolerance (north_star): <= 1e-12 relative FP64, measured as max|du|/max|u| and ||du||_2/||u||_2."""
+import os
+
 import numpy as np
 import pytest
 
 import oracle as orc
 import skellysim_b200 as skb
-from conftest import rel_l2, rel_max
+from conftest import GOLDEN_DIR, rel_l2, rel_max
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-12
@@ -63,12 +65,11 @@ def test_golden_reference_outputs(golden_cases, case):
 
 
 def test_against_reference_cuda_kernels():
-    # the UNMODIFIED reference kernels.cu, run on this GPU, vs the oracle and vs the new path
-    if not orc.refgpu_available():
-        pytest.fail("oracle/_ref/libskelly_ref_kernels_cu.so missing: run `make -C oracle` in the build container")
-    rs, rt, f3, f9 = _rand(21, 1229, 743, coincident=17)
-    ref_u = orc.ref_stokeslet_direct_gpu_impl(rs, f3, rt)
-    ref_d = orc.ref_stresslet_direct_gpu_impl(rs, f9, rt)
+    # the UNMODIFIED reference kernels.cu, run on a B200 (stored by tests/golden/make_golden.py --cuda), vs the oracle
+    # and vs the new path
+    g = np.load(os.path.join(GOLDEN_DIR, "ref_cuda_kernels.npz"))
+    rs, rt, f3, f9 = g["r_src"], g["r_trg"], g["f_sl"], g["f_dl"]
+    ref_u, ref_d = g["u_stokeslet"], g["u_stresslet"]
     # oracle pinned by the reference itself
     _check(orc.stokeslet_direct(rs, f3, rt), ref_u)
     _check(orc.stresslet_direct(rs, f9, rt), ref_d)
